@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the marlbase hot path on B200 (BASELINE.json metric) next to the CPU reference loop.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config idqn|vdn15|ia2c]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config idqn|vdn15|ia2c] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Default workload (`--config idqn`) = BASELINE.json configs[1], the configuration the metric is quoted on: IDQN on
@@ -43,6 +43,7 @@ WORKLOADS = {
 TRAFFIC_NCU = {"tc_dqn_fwd_kernel": 9303552, "tc_dh1_kernel": 3705344, "tc_dw_kernel": 92672512,
                # on-chip pass (round 2): dram__bytes of one launch inside the running pipeline (ncu --cache-control none, profiles/r2_dram_traffic.md)
                "tc_dqn_fwd3_kernel": 4300000, "tc_dh1w1_kernel": 10300000, "tc_dw2_kernel": 10300000}
+DUMP_EPISODES = 1024   # --dump-outputs: episodes of the last step kept (a fixed, seeded sample), so that the files stay small at any --envs
 
 
 def parse():
@@ -63,7 +64,12 @@ def parse():
                     help="N > 1: gradient exchange inside the fused reduce + Adam kernel over NVLink peer memory (default), or one NCCL all-reduce per update")
     ap.add_argument("--tc-backward", type=int, default=1, help="1 = tcgen05 training pipeline (default), 0 = fused FP32 FFMA training kernel")
     ap.add_argument("--tc-onchip", type=int, default=1, help="1 = training pass with H1 / H2 / dH1 kept on chip (tc_train3.cu, default), 0 = streamed through global memory (tc_train.cu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32): parameters, target parameters, update "
+                         f"metrics, every env's episode length and return, and a fixed sample of at most {DUMP_EPISODES} of the episodes it collected")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     wl = WORKLOADS[a.config]
     a.envs = a.envs or wl["envs"]
     a.batch = a.batch or wl["batch"]
@@ -240,6 +246,7 @@ class Harness:
         if not torch.cuda.is_available():
             raise SystemExit("bench.py: no CUDA device -- the B200 path has no CPU fallback")
         torch.cuda.set_device(self.local)
+        torch.manual_seed(args.seed)   # the networks' initialisation: with the same arguments every run computes the same (--dump-outputs)
         self.dev = torch.device("cuda", self.local)
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
@@ -271,6 +278,23 @@ class Harness:
     def finish(self):
         if self.world > 1:
             self.dist.destroy_process_group()
+
+
+def dump_outputs(torch, out_dir, model, nat_env, store, slot0):
+    """--dump-outputs: what the last timed step computed -- the parameters and target parameters after its updates, the metrics of its last update,
+    each env's episode length and return, and a fixed, seeded sample of the episodes it wrote to `store` from slot `slot0` on -- as float32 .npy files."""
+    import numpy as np
+
+    E = nat_env.E
+    pick = np.sort(np.random.default_rng(0).choice(E, min(E, DUMP_EPISODES), replace=False))
+    slots = torch.as_tensor((slot0 + pick) % store.capacity, device=store.obs.device)
+    arrays = {"theta": model.theta, "theta_target": model.theta_tgt, "metrics": model._metrics, "episode_length": nat_env.final_len,
+              "episode_return": nat_env.final_ret, "episode_index": pick}
+    arrays.update({f"episodes_{k}": getattr(store, k)[slots] for k in ("obs", "act", "rew", "done", "filled")})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else t
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
 
 
 def theta_fingerprint(torch, theta):
@@ -374,6 +398,8 @@ def run_dqn_family(args, wl):
     sampler = ClockSampler(H.local) if rank == 0 else None
     ms, n_steps = H.timed(args.steps, lambda: iteration(False))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, model, nat_env, rb, (state["pos"] - E) % args.buffer)
 
     # ---- multi-GPU correctness, driver visible: replicated parameters must be BIT-identical on every rank after the timed region, and the in-kernel
     # peer-memory exchange must agree with the plain NCCL all-reduce path on one update from the same state (tests/test_peer_exchange_gpu.py asserts
@@ -569,6 +595,8 @@ def run_ia2c(args, wl):
     sampler = ClockSampler(H.local) if rank == 0 else None
     ms, n_steps = H.timed(args.steps, lambda: iteration(False))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, model, nat_env, b, 0)
     multi = None
     if world > 1:
         fp = theta_fingerprint(torch, model.theta)

@@ -1,8 +1,8 @@
 """CPU restatement (PyTorch float32, autograd) of the reference learner arithmetic.  TEST INFRASTRUCTURE ONLY.
 
 Written functionally over FLAT parameter vectors in the device layout ([n_nets][P], reference state_dict order), so
-that it also pins the layout conversion.  Pinned against the live reference classes (tests marked `refsrc`, build
-container only) and against committed golden vectors generated from them (tests/golden/, make_golden.py).
+that it also pins the layout conversion.  Pinned against committed golden vectors generated from the live reference
+classes (tests/golden/: make_golden.py and the make_reference_cases functions of the tests).
 
 Restated from (path:line under /root/reference/marlbase):
   utils/models.py:14-48      FCNetwork = Linear-ReLU-Linear-ReLU-Linear

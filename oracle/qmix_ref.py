@@ -9,7 +9,7 @@ Restated from (path:line under /root/reference/marlbase):
 The mixer's parameters are one flat vector in the reference's state_dict order (hypernet_layers == 2):
   hyper_w_1.0.{weight [He,S], bias [He]}, hyper_w_1.2.{weight [N*E,He], bias [N*E]}, hyper_w_final.0.{weight [He,S], bias [He]},
   hyper_w_final.2.{weight [E,He], bias [E]}, hyper_b_1.{weight [E,S], bias [E]}, V.0.{weight [E,S], bias [E]}, V.2.{weight [1,E], bias [1]}
-Pinned against the live reference classes by tests/test_qmix.py (refsrc tests, build container) and the golden vectors it checks.
+Pinned by tests/test_qmix.py against outputs of the live reference classes recorded under tests/golden/ (ref_qmix.npz, qmix_indep.npz).
 """
 from __future__ import annotations
 

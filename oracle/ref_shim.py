@@ -1,9 +1,11 @@
-"""Import shim for the LIVE reference learner classes under /root/reference (build container only).
+"""Import shim for the LIVE reference learner classes of a marlbase checkout (the directory that holds `marlbase/`, named by the
+MARLBASE_SRC environment variable).
 
 TEST INFRASTRUCTURE ONLY.  The reference's learner half imports cleanly once `gymnasium.spaces.flatdim`
 (its only gymnasium use: marlbase/dqn/model.py:4, marlbase/ac/model.py:4) and stub `hydra` / `omegaconf` /
-`imageio` modules exist (imports at marlbase/dqn/train.py:6,8,11).  Nothing here is available on the GPU box:
-tests that use it are marked `refsrc`, and tests/golden/make_golden.py uses it to emit committed fixtures.
+`imageio` modules exist (imports at marlbase/dqn/train.py:6,8,11).  The test suite never needs it: the fixture
+generators (tests/golden/make_golden.py and the `make_*` functions of the test modules) use it to record what the
+reference computes into the committed files under tests/golden/.
 """
 from __future__ import annotations
 
@@ -11,11 +13,11 @@ import os
 import sys
 import types
 
-REF_ROOT = "/root/reference"
+REF_ROOT = os.environ.get("MARLBASE_SRC", "")
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REF_ROOT, "marlbase"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "marlbase"))
 
 
 class Space:
@@ -39,7 +41,7 @@ def _flatdim(space):
 def load():
     """Returns a namespace with the reference modules: dqn_model, dqn_train, ac_model, utils, models."""
     if not available():
-        raise RuntimeError("/root/reference is not present")
+        raise RuntimeError("set MARLBASE_SRC to a directory that contains the marlbase package")
     if "gymnasium" not in sys.modules:
         gym = types.ModuleType("gymnasium")
         spaces = types.ModuleType("gymnasium.spaces")

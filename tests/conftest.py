@@ -10,14 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu on the GPU box")
-    config.addinivalue_line("markers", "refsrc: needs /root/reference (only present in the build container)")
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/marlbase")
-    for item in items:
-        if "refsrc" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference is not present on this box"))
 
 
 @pytest.fixture(autouse=True)

@@ -1,5 +1,5 @@
-"""Generates tests/golden/*.npz from the LIVE reference learner classes (build container only; /root/reference does
-not exist on the GPU box).  Run:  python tests/golden/make_golden.py
+"""Generates the learner fixtures under tests/golden/ from the LIVE reference learner classes of a marlbase checkout.
+Run:  MARLBASE_SRC=<directory holding marlbase/> python tests/golden/make_golden.py
 Every fixture stores the inputs in the device ("trajectory store") layout plus the reference's outputs, so that both
 the CPU oracle (oracle/learner_ref.py) and the CUDA path are checked against numbers the reference itself produced."""
 import os

@@ -35,6 +35,33 @@ def assert_grad_close(lr, st, batch, hp, got, want, tol=1e-5, what=""):
     raise AssertionError(f"{what} max abs error {err:.3e} > {tol:g} x {scale:.3g} (largest ReLU-kink move of this case: {risk:.3e})")
 
 
+def net_layers(n_nets, in_dim, out_dim, hidden=128):
+    """(out, in) of every Linear layer of `n_nets` FCNetworks, in the order of the flat parameter vector."""
+    return [(hidden, in_dim), (hidden, hidden), (out_dim, hidden)] * n_nets
+
+
+def sample_index(layers, per_tensor=64):
+    """Positions at which the recorded reference outputs (tests/golden/ref_*.npz) keep a flat parameter vector made of consecutive Linear layers
+    (weight, then bias): at most `per_tensor` evenly spaced elements of every weight and every bias, so that each tensor is checked while the files
+    stay small."""
+    import numpy as np
+
+    out, o = [], 0
+    for no, ni in layers:
+        for n in (no * ni, no):
+            out.append(o + np.unique(np.linspace(0, n - 1, min(n, per_tensor)).round().astype(np.int64)))
+            o += n
+    return np.concatenate(out)
+
+
+def load_case(path, case):
+    """The arrays of one recorded case (keys `<case>.<name>`) of a tests/golden/ref_*.npz file."""
+    import numpy as np
+
+    with np.load(path) as g:
+        return {k[len(case) + 1:]: g[k] for k in g.files if k.startswith(case + ".")}
+
+
 def redraw_on_near_tie(fn):
     """Run the test body with seeds 0, 1, ... until its oracle argmax margin is healthy (at most five draws): with a healthy margin every mismatch
     is a defect; five near-ties in a row are not plausible (they occur in ~8 % of random initialisations, tools/grad_stress.py)."""

@@ -1,6 +1,5 @@
-"""CPU: oracle/learner_ref.py (the torch-CPU restatement that travels to the GPU box) pinned against golden vectors
-produced by the LIVE reference classes (tests/golden/make_golden.py) and, when /root/reference is present, against
-the live classes directly."""
+"""CPU: oracle/learner_ref.py (the torch-CPU restatement the GPU tests compare against) pinned against golden vectors
+produced by the LIVE reference classes (tests/golden/make_golden.py, make_reference_cases below)."""
 import os
 
 import numpy as np
@@ -8,6 +7,7 @@ import pytest
 import torch
 
 from oracle import learner_ref as lr
+from tests.helpers import load_case, net_layers, sample_index
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 N, D, A, T = 2, 15, 6, 25
@@ -92,52 +92,85 @@ def test_epsilon_schedule_and_nstep_returns_golden():
         _close(got.numpy(), g[f"ns_ret_{n}"], rtol=1e-6, atol=1e-6)
 
 
-@pytest.mark.refsrc
-def test_replay_ring_matches_live_reference_buffer():
-    """ReplayRef (episode-major) == reference ReplayBuffer (time-major) incl. the stale tail of re-used slots."""
-    from oracle import ref_shim
+LIVE = os.path.join(GOLD, "ref_oracle_learner.npz")
 
-    ref = ref_shim.load()
-    rng = np.random.default_rng(1)
-    spaces = [ref_shim.Space(shape=(D,)) for _ in range(N)]
-    rb = ref.dqn_train.ReplayBuffer(5, N, spaces, [ref_shim.Space(n=A)] * N, T, "cpu")
-    mine = lr.ReplayRef(5, N, T, D)
-    for ep in range(12):
+
+def _replay_episodes(rng):
+    """12 episodes of random lengths into a 5-slot ring: (first observations, [(observations, actions, rewards, done) per step]) per episode"""
+    for _ in range(12):
         L = int(rng.integers(2, T + 1))
-        o = [rng.standard_normal(D).astype(np.float32) for _ in range(N)]
-        rb.init_episode(o); mine.init_episode(o)
+        o0 = [rng.standard_normal(D).astype(np.float32) for _ in range(N)]
+        steps = []
         for t in range(L):
             o = [rng.standard_normal(D).astype(np.float32) for _ in range(N)]
-            a, r, d = rng.integers(0, A, N), rng.random(N).astype(np.float32), t == L - 1
-            rb.add(o, a, r, d); mine.add(o, a, r, d)
-    assert len(rb) == len(mine) and rb.cur_pos == mine.cur
-    for i in range(N):
-        assert np.array_equal(rb.observations[i].transpose(1, 0, 2), mine.store["obs"][:, i])
-    assert np.array_equal(rb.actions.transpose(2, 0, 1), mine.store["act"])
-    assert np.array_equal(rb.rewards.transpose(2, 0, 1), mine.store["rew"])
-    assert np.array_equal(rb.dones.T, mine.store["done"].astype(bool)) and np.array_equal(rb.filled.T, mine.store["filled"].astype(bool))
+            steps.append((o, rng.integers(0, A, N), rng.random(N).astype(np.float32), t == L - 1))
+        yield o0, steps
 
 
-@pytest.mark.refsrc
-def test_live_reference_update_on_fresh_seed():
-    """Not only the committed vectors: a fresh random case against the live classes."""
+def _fresh_batch(rng, B=16):
+    return dict(obss=torch.tensor(rng.standard_normal((N, T + 1, B, D)), dtype=torch.float32), actions=torch.tensor(rng.integers(0, A, (N, T, B))),
+                rewards=torch.tensor(rng.random((N, T, B)), dtype=torch.float32), dones=torch.tensor(rng.random((T + 1, B)) < 0.05, dtype=torch.float32),
+                filled=torch.tensor(rng.random((T, B)) < 0.9, dtype=torch.float32))
+
+
+def make_reference_cases():
+    """Records tests/golden/ref_oracle_learner.npz from the reference's ReplayBuffer and QNetwork: MARLBASE_SRC=<marlbase checkout> python -c 'import
+    tests.test_oracle_learner as t; t.make_reference_cases()'."""
     from oracle import ref_shim
 
     ref = ref_shim.load()
+    rb = ref.dqn_train.ReplayBuffer(5, N, [ref_shim.Space(shape=(D,)) for _ in range(N)], [ref_shim.Space(n=A)] * N, T, "cpu")
+    for o0, steps in _replay_episodes(np.random.default_rng(1)):
+        rb.init_episode(o0)
+        for o, a, r, d in steps:
+            rb.add(o, a, r, d)
+    out = {"ring.len": np.int64(len(rb)), "ring.cur_pos": np.int64(rb.cur_pos), "ring.actions": rb.actions, "ring.rewards": rb.rewards,
+           "ring.dones": rb.dones, "ring.filled": rb.filled, "ring.observations": np.stack(rb.observations)}
     torch.manual_seed(123)
     model = ref.dqn_model.QNetwork([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, ref_shim.dqn_cfg(), [128, 128], False, False, True, "cpu")
-    theta = lr.flat_from_state_dict(model.state_dict(), "critic.independent", N)
+    idx = sample_index(net_layers(N, D, A))
+    out["fresh.theta0"] = lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy()[idx]
+    rng = np.random.default_rng(4)
+    losses = []
+    for _ in range(2):
+        b = _fresh_batch(rng)
+        losses.append(model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"])
+    out["fresh.loss"] = np.array(losses, np.float64)
+    out["fresh.theta"] = lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy()[idx]
+    np.savez_compressed(LIVE, **out)
+
+
+def test_replay_ring_matches_live_reference_buffer():
+    """ReplayRef (episode-major) == reference ReplayBuffer (time-major, recorded in tests/golden/ref_oracle_learner.npz) incl. the stale tail of
+    re-used slots."""
+    rb = load_case(LIVE, "ring")
+    mine = lr.ReplayRef(5, N, T, D)
+    for o0, steps in _replay_episodes(np.random.default_rng(1)):
+        mine.init_episode(o0)
+        for o, a, r, d in steps:
+            mine.add(o, a, r, d)
+    assert int(rb["len"]) == len(mine) and int(rb["cur_pos"]) == mine.cur
+    for i in range(N):
+        assert np.array_equal(rb["observations"][i].transpose(1, 0, 2), mine.store["obs"][:, i])
+    assert np.array_equal(rb["actions"].transpose(2, 0, 1), mine.store["act"])
+    assert np.array_equal(rb["rewards"].transpose(2, 0, 1), mine.store["rew"])
+    assert np.array_equal(rb["dones"].T, mine.store["done"].astype(bool)) and np.array_equal(rb["filled"].T, mine.store["filled"].astype(bool))
+
+
+def test_live_reference_update_on_fresh_seed():
+    """Not only the fixtures of make_golden.py: a further random case (the reference's default DQN settings, torch seed 123) against what the
+    reference's QNetwork computed (tests/golden/ref_oracle_learner.npz)."""
+    g = load_case(LIVE, "fresh")
+    idx = sample_index(net_layers(N, D, A))
+    torch.manual_seed(123)
+    theta = lr.init_flat(N, D, A)
+    assert np.abs(theta.numpy()[idx] - g["theta0"]).max() < 1e-6, "initialisation differs from the reference's"
     st = lr.DqnState(theta.clone(), theta.clone(), [0, 1], D, A)
     rng = np.random.default_rng(4)
-    for _ in range(2):
-        B = 16
-        b = dict(obss=torch.tensor(rng.standard_normal((N, T + 1, B, D)), dtype=torch.float32), actions=torch.tensor(rng.integers(0, A, (N, T, B))),
-                 rewards=torch.tensor(rng.random((N, T, B)), dtype=torch.float32), dones=torch.tensor(rng.random((T + 1, B)) < 0.05, dtype=torch.float32),
-                 filled=torch.tensor(rng.random((T, B)) < 0.9, dtype=torch.float32))
-        want = model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"]
-        got = lr.dqn_update(st, b, lr.DqnHP())
+    for want in g["loss"]:
+        got = lr.dqn_update(st, _fresh_batch(rng), lr.DqnHP())
         _close(got["loss"], want)
-    d = np.abs(st.theta.numpy() - lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy())
+    d = np.abs(st.theta.numpy()[idx] - g["theta"])
     assert np.quantile(d, 0.999) < 1e-5
 
 

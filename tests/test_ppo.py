@@ -1,5 +1,6 @@
-"""IPPO (marlbase/ac/model.py PPONetwork, 249-352): the oracle restatement against the LIVE reference class (build container only, `refsrc`),
+"""IPPO (marlbase/ac/model.py PPONetwork, 249-352): the oracle restatement against recorded outputs of the reference classes (tests/golden/ref_ppo.npz),
 and the B200 path (marl_ppo_update through ac.model.PPONetwork) against the oracle on random on-policy batches; driver test."""
+import os
 import types
 
 import numpy as np
@@ -7,6 +8,7 @@ import pytest
 import torch
 
 from oracle import learner_ref as lr
+from tests.helpers import load_case, net_layers, sample_index
 
 N, D, A, T = 2, 15, 6, 25
 
@@ -39,93 +41,123 @@ def _oracle_batch(s):
                 rewards=t["rew"].permute(2, 0, 1).float(), dones=t["done"].permute(1, 0).float(), filled=t["filled"].permute(1, 0).float())
 
 
-@pytest.mark.refsrc
+METRICS = ("loss", "actor_loss", "value_loss", "entropy")
+LIVE = os.path.join(os.path.dirname(__file__), "golden", "ref_ppo.npz")
+# the reference runs recorded by make_reference_cases: name -> (class, torch seed, batch seed, envs per batch, update steps, config, critic config)
+LIVE_CASES = {
+    "std_A2CNetwork": ("A2CNetwork", 9, 3, 10, (0, 2, 3), dict(standardise_returns=True, num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2), {}),
+    "std_PPONetwork": ("PPONetwork", 9, 3, 10, (0, 2, 3), dict(standardise_returns=True, num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2), {}),
+    "cent_A2CNetwork": ("A2CNetwork", 4, 5, 10, (0, 2, 3), dict(num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2), dict(centralised=True)),
+    "cent_PPONetwork": ("PPONetwork", 4, 5, 10, (0, 2, 3), dict(num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2), dict(centralised=True)),
+    "ppo_indep_noclip": ("PPONetwork", 5, 11, 12, (0, 2, 5), dict(grad_clip=False, num_epochs=4, ppo_clip=0.2, target_update_interval_or_tau=2), {}),
+    "ppo_shared_clip": ("PPONetwork", 5, 11, 12, (0, 2, 5), dict(grad_clip=0.5, num_epochs=4, ppo_clip=0.2, target_update_interval_or_tau=2), dict(parameter_sharing=True)),
+}
+
+
+def _live_layout(case):
+    """(n_nets, critic input width, sample positions of the actor, of the critic) of a recorded case"""
+    crit = LIVE_CASES[case][6]
+    n_nets = 1 if crit.get("parameter_sharing") else N
+    c_in = N * D if crit.get("centralised") else D
+    return n_nets, c_in, sample_index(net_layers(n_nets, D, A)), sample_index(net_layers(n_nets, c_in, 1))
+
+
+def make_reference_cases():
+    """Records tests/golden/ref_ppo.npz from the reference's A2CNetwork / PPONetwork: MARLBASE_SRC=<marlbase checkout> python -c 'import
+    tests.test_ppo as t; t.make_reference_cases()'.  Per case: the metrics of each update, the return statistics, and the parameters before and after
+    at the positions of _live_layout."""
+    from collections import namedtuple
+
+    from oracle import ref_shim
+
+    ref = ref_shim.load()
+    Batch = namedtuple("Batch", ["obss", "actions", "rewards", "dones", "filled", "action_masks"])
+    out = {}
+    for case, (cls, seed, bseed, P, steps, cfgkw, critkw) in LIVE_CASES.items():
+        n_nets, c_in, ia, ic = _live_layout(case)
+        kind = "networks" if n_nets == 1 else "independent"
+        torch.manual_seed(seed)
+        net = ref_shim.net_cfg(parameter_sharing=bool(critkw.get("parameter_sharing")))
+        model = getattr(ref.ac_model, cls)([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, ref_shim.a2c_cfg(**cfgkw), net, ref_shim.net_cfg(**critkw), "cpu")
+        sd = model.state_dict()
+        out[f"{case}.critic_in"] = np.int64(sd[f"critic.{kind}.0.network.0.weight"].shape[1])
+        out[f"{case}.actor0"] = lr.flat_from_state_dict(sd, f"actor.{kind}", n_nets).numpy()[ia]
+        out[f"{case}.critic0"] = lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets).numpy()[ic]
+        out[f"{case}.target0"] = lr.flat_from_state_dict(sd, f"target_critic.{kind}", n_nets).numpy()[ic]
+        rng = np.random.default_rng(bseed)
+        metrics = []
+        for step in steps:
+            b = _oracle_batch(_batch_arrays(rng, P, N))
+            want = model.update(Batch(b["obss"], b["actions"], b["rewards"], b["dones"].bool(), b["filled"], None), step)
+            metrics.append([want[k] for k in METRICS])
+        out[f"{case}.metrics"] = np.array(metrics, np.float64)
+        if cfgkw.get("standardise_returns"):
+            out.update({f"{case}.ret_mean": model.ret_ms.mean.numpy(), f"{case}.ret_var": model.ret_ms.var.numpy(), f"{case}.ret_count": np.float64(model.ret_ms.count)})
+        sd = model.state_dict()
+        out.update({f"{case}.actor": lr.flat_from_state_dict(sd, f"actor.{kind}", n_nets).numpy()[ia],
+                    f"{case}.critic": lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets).numpy()[ic],
+                    f"{case}.target": lr.flat_from_state_dict(sd, f"target_critic.{kind}", n_nets).numpy()[ic]})
+    np.savez_compressed(LIVE, **out)
+
+
+def _live_state(case, g, **kw):
+    """The oracle's state from the reference's initialisation (torch seed of the case; actor drawn before critic, the target critic is a copy)"""
+    n_nets, c_in, ia, ic = _live_layout(case)
+    assert int(g["critic_in"]) == c_in
+    torch.manual_seed(LIVE_CASES[case][1])
+    actor, critic = lr.init_flat(n_nets, D, A), lr.init_flat(n_nets, c_in, 1)
+    for mine, key, idx in ((actor, "actor0", ia), (critic, "critic0", ic), (critic, "target0", ic)):
+        assert np.abs(mine.numpy()[idx] - g[key]).max() < 1e-6, f"initialisation differs from the reference's ({key})"
+    nets = [0] * N if n_nets == 1 else list(range(N))
+    return lr.A2CState(actor, critic, critic.clone(), nets, nets, D, A, **kw), ia, ic
+
+
+def _run_live_case(case, st, update):
+    g = load_case(LIVE, case)
+    rng = np.random.default_rng(LIVE_CASES[case][2])
+    for step, want in zip(LIVE_CASES[case][4], g["metrics"]):
+        got = update(st, _oracle_batch(_batch_arrays(rng, LIVE_CASES[case][3], N)), step)
+        _close([got[k] for k in METRICS], want)
+    return g
+
+
 @pytest.mark.parametrize("cls", ["A2CNetwork", "PPONetwork"])
 def test_oracle_standardise_returns_matches_live_reference(cls):
-    """cfg.standardise_returns=True: RunningMeanStd over the n-step returns (ac/model.py:195-204, 272-281) -- oracle vs the live classes"""
-    from collections import namedtuple
-
-    from oracle import ref_shim
-
-    ref = ref_shim.load()
-    torch.manual_seed(9)
-    cfg = ref_shim.a2c_cfg(standardise_returns=True, num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2)
-    net = ref_shim.net_cfg()
-    model = getattr(ref.ac_model, cls)([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, cfg, net, net, "cpu")
-    sd = model.state_dict()
-    st = lr.A2CState(lr.flat_from_state_dict(sd, "actor.independent", N), lr.flat_from_state_dict(sd, "critic.independent", N),
-                     lr.flat_from_state_dict(sd, "target_critic.independent", N), [0, 1], [0, 1], D, A, ret_ms=lr.RunningMeanStdRef((N,)))
+    """cfg.standardise_returns=True: RunningMeanStd over the n-step returns (ac/model.py:195-204, 272-281) -- oracle vs what the reference's classes
+    computed (tests/golden/ref_ppo.npz)"""
+    case = f"std_{cls}"
+    st, ia, _ = _live_state(case, load_case(LIVE, case), ret_ms=lr.RunningMeanStdRef((N,)))
     hp = lr.A2CHP(target_update_interval_or_tau=2)
-    Batch = namedtuple("Batch", ["obss", "actions", "rewards", "dones", "filled", "action_masks"])
-    rng = np.random.default_rng(3)
-    for step in (0, 2, 3):
-        b = _oracle_batch(_batch_arrays(rng, 10, N))
-        want = model.update(Batch(b["obss"], b["actions"], b["rewards"], b["dones"].bool(), b["filled"], None), step)
-        got = lr.ppo_update(st, b, hp, step, 3, 0.2) if cls == "PPONetwork" else lr.a2c_update(st, b, hp, step)
-        _close([got[k] for k in ("loss", "actor_loss", "value_loss", "entropy")], [want[k] for k in ("loss", "actor_loss", "value_loss", "entropy")])
-    _close(st.ret_ms.mean.numpy(), model.ret_ms.mean.numpy()); _close(st.ret_ms.var.numpy(), model.ret_ms.var.numpy())
-    assert abs(st.ret_ms.count - model.ret_ms.count) < 1e-9
-    d = np.abs(st.actor.numpy() - lr.flat_from_state_dict(model.state_dict(), "actor.independent", N).numpy())
+    g = _run_live_case(case, st, lambda st, b, step: lr.ppo_update(st, b, hp, step, 3, 0.2) if cls == "PPONetwork" else lr.a2c_update(st, b, hp, step))
+    _close(st.ret_ms.mean.numpy(), g["ret_mean"]); _close(st.ret_ms.var.numpy(), g["ret_var"])
+    assert abs(st.ret_ms.count - float(g["ret_count"])) < 1e-9
+    d = np.abs(st.actor.numpy()[ia] - g["actor"])
     assert np.quantile(d, 0.999) < 1e-5
 
 
-@pytest.mark.refsrc
 @pytest.mark.parametrize("cls", ["A2CNetwork", "PPONetwork"])
 def test_oracle_centralised_critic_matches_live_reference(cls):
-    """critic.centralised=True (MAA2C / MAPPO, ac/model.py:62-65,156-157): oracle vs the live classes"""
-    from collections import namedtuple
-
-    from oracle import ref_shim
-
-    ref = ref_shim.load()
-    torch.manual_seed(4)
-    cfg = ref_shim.a2c_cfg(num_epochs=3, ppo_clip=0.2, target_update_interval_or_tau=2)
-    model = getattr(ref.ac_model, cls)([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, cfg, ref_shim.net_cfg(), ref_shim.net_cfg(centralised=True), "cpu")
-    sd = model.state_dict()
-    assert sd["critic.independent.0.network.0.weight"].shape == (128, N * D)
-    st = lr.A2CState(lr.flat_from_state_dict(sd, "actor.independent", N), lr.flat_from_state_dict(sd, "critic.independent", N),
-                     lr.flat_from_state_dict(sd, "target_critic.independent", N), [0, 1], [0, 1], D, A, centralised=True)
+    """critic.centralised=True (MAA2C / MAPPO, ac/model.py:62-65,156-157): oracle vs what the reference's classes computed (tests/golden/ref_ppo.npz)"""
+    case = f"cent_{cls}"
+    st, _, ic = _live_state(case, load_case(LIVE, case), centralised=True)
     hp = lr.A2CHP(target_update_interval_or_tau=2)
-    Batch = namedtuple("Batch", ["obss", "actions", "rewards", "dones", "filled", "action_masks"])
-    rng = np.random.default_rng(5)
-    for step in (0, 2, 3):
-        b = _oracle_batch(_batch_arrays(rng, 10, N))
-        want = model.update(Batch(b["obss"], b["actions"], b["rewards"], b["dones"].bool(), b["filled"], None), step)
-        got = lr.ppo_update(st, b, hp, step, 3, 0.2) if cls == "PPONetwork" else lr.a2c_update(st, b, hp, step)
-        _close([got[k] for k in ("loss", "actor_loss", "value_loss", "entropy")], [want[k] for k in ("loss", "actor_loss", "value_loss", "entropy")])
-    d = np.abs(st.critic.numpy() - lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy())
+    g = _run_live_case(case, st, lambda st, b, step: lr.ppo_update(st, b, hp, step, 3, 0.2) if cls == "PPONetwork" else lr.a2c_update(st, b, hp, step))
+    d = np.abs(st.critic.numpy()[ic] - g["critic"])
     assert np.quantile(d, 0.999) < 1e-5
 
 
-@pytest.mark.refsrc
 @pytest.mark.parametrize("sharing,clip", [(False, False), (True, 0.5)])
 def test_oracle_ppo_matches_live_reference(sharing, clip):
-    """three PPO updates (4 epochs each) of the reference's PPONetwork vs oracle.learner_ref.ppo_update from the same weights and batches"""
-    from collections import namedtuple
-
-    from oracle import ref_shim
-
-    ref = ref_shim.load()
-    torch.manual_seed(5)
-    cfg = ref_shim.a2c_cfg(grad_clip=clip, num_epochs=4, ppo_clip=0.2, target_update_interval_or_tau=2)
-    net = ref_shim.net_cfg(parameter_sharing=sharing)
-    model = ref.ac_model.PPONetwork([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, cfg, net, net, "cpu")
-    kind, n_nets, nets = ("networks", 1, [0, 0]) if sharing else ("independent", N, [0, 1])
-    sd = model.state_dict()
-    st = lr.A2CState(lr.flat_from_state_dict(sd, f"actor.{kind}", n_nets), lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets),
-                     lr.flat_from_state_dict(sd, f"target_critic.{kind}", n_nets), nets, nets, D, A)
+    """three PPO updates (4 epochs each) of oracle.learner_ref.ppo_update vs what the reference's PPONetwork computed from the same weights and
+    batches (tests/golden/ref_ppo.npz)"""
+    case = "ppo_shared_clip" if sharing else "ppo_indep_noclip"
+    assert LIVE_CASES[case][5]["grad_clip"] == clip
+    st, ia, ic = _live_state(case, load_case(LIVE, case))
     hp = lr.A2CHP(grad_clip=float(clip or 0.0), target_update_interval_or_tau=2)
-    Batch = namedtuple("Batch", ["obss", "actions", "rewards", "dones", "filled", "action_masks"])
-    rng = np.random.default_rng(11)
-    for step in (0, 2, 5):
-        b = _oracle_batch(_batch_arrays(rng, 12, N))
-        want = model.update(Batch(b["obss"], b["actions"], b["rewards"], b["dones"].bool(), b["filled"], None), step)
-        got = lr.ppo_update(st, b, hp, step, 4, 0.2)
-        _close([got[k] for k in ("loss", "actor_loss", "value_loss", "entropy")], [want[k] for k in ("loss", "actor_loss", "value_loss", "entropy")])
-    sd = model.state_dict()
-    for mine, prefix in ((st.actor, f"actor.{kind}"), (st.critic, f"critic.{kind}"), (st.target, f"target_critic.{kind}")):
-        d = np.abs(mine.numpy() - lr.flat_from_state_dict(sd, prefix, n_nets).numpy())
-        assert np.quantile(d, 0.999) < 1e-5, (prefix, d.max())
+    g = _run_live_case(case, st, lambda st, b, step: lr.ppo_update(st, b, hp, step, 4, 0.2))
+    for mine, key, idx in ((st.actor, "actor", ia), (st.critic, "critic", ic), (st.target, "target", ic)):
+        d = np.abs(mine.numpy()[idx] - g[key])
+        assert np.quantile(d, 0.999) < 1e-5, (key, d.max())
 
 
 def test_oracle_ppo_first_epoch_is_a2c_with_unit_ratio():

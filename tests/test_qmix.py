@@ -1,5 +1,5 @@
-"""QMIX (marlbase/dqn/model.py:272-443): the oracle restatement against the live reference and a committed golden vector (CPU), the CUDA mixer
-against the oracle (GPU)."""
+"""QMIX (marlbase/dqn/model.py:272-443): the oracle restatement against recorded outputs of the reference and a committed golden vector (CPU), the
+CUDA mixer against the oracle (GPU)."""
 import os
 
 import numpy as np
@@ -8,7 +8,7 @@ import torch
 
 from oracle import learner_ref as lr
 from oracle import qmix_ref as qr
-from tests.helpers import NearTie, redraw_on_near_tie
+from tests.helpers import NearTie, load_case, net_layers, redraw_on_near_tie, sample_index
 
 N, T, D, A = 2, 6, 9, 6
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "qmix_indep.npz")
@@ -35,32 +35,67 @@ def _state_from(model, sharing=False):
     return qr.QmixState(theta.clone(), theta.clone(), mix.clone(), mix.clone(), [0] * N if sharing else list(range(N)), D, A)
 
 
-@pytest.mark.refsrc
-@pytest.mark.parametrize("tu,sharing", [(2.0, False), (0.05, False), (2.0, True)])
-def test_oracle_matches_live_reference(tu, sharing):
+LIVE_CASES = [(2.0, False), (0.05, False), (2.0, True)]
+LIVE = os.path.join(os.path.dirname(__file__), "golden", "ref_qmix.npz")
+
+
+def _live_index(sharing):
+    return sample_index(net_layers(1 if sharing else N, D, A)), sample_index(qr.mixer_shapes(N, N * D, 64, 32))
+
+
+def make_reference_cases():
+    """Records tests/golden/ref_qmix.npz from the reference's QMixNetwork: MARLBASE_SRC=<marlbase checkout> python -c 'import tests.test_qmix as t;
+    t.make_reference_cases()'.  Per case: the loss of each of three updates and the four parameter sets after them at the positions of _live_index."""
     from oracle import ref_shim
 
     ref = ref_shim.load()
-    torch.manual_seed(11)
-    model = _ref_model(ref, ref_shim, tu, sharing)
-    st = _state_from(model, sharing)
-    kind, n_nets = ("networks", 1) if sharing else ("independent", N)
-    assert st.mix.numel() == qr.mixer_size(N, N * D, 64, 32)
+    out = {}
+    for c, (tu, sharing) in enumerate(LIVE_CASES):
+        torch.manual_seed(11)
+        model = _ref_model(ref, ref_shim, tu, sharing)
+        kind, n_nets = ("networks", 1) if sharing else ("independent", N)
+        it, im = _live_index(sharing)
+        sd = model.state_dict()
+        out.update({f"c{c}.theta0": lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets).numpy()[it], f"c{c}.mix0": qr.mixer_flat_from_state_dict(sd, "mixer").numpy()[im],
+                    f"c{c}.n_mix": np.int64(qr.mixer_flat_from_state_dict(sd, "mixer").numel())})
+        rng = np.random.default_rng(5)
+        losses = []
+        for _ in range(3):
+            b = _batch(rng, 16)
+            losses.append(model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"])
+        sd = model.state_dict()
+        out.update({f"c{c}.loss": np.array(losses, np.float64), f"c{c}.theta": lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets).numpy()[it],
+                    f"c{c}.theta_tgt": lr.flat_from_state_dict(sd, f"target.{kind}", n_nets).numpy()[it],
+                    f"c{c}.mix": qr.mixer_flat_from_state_dict(sd, "mixer").numpy()[im], f"c{c}.mix_tgt": qr.mixer_flat_from_state_dict(sd, "target_mixer").numpy()[im]})
+    np.savez_compressed(LIVE, **out)
+
+
+@pytest.mark.parametrize("tu,sharing", LIVE_CASES)
+def test_oracle_matches_live_reference(tu, sharing):
+    """Three updates of the oracle against what the reference's QMixNetwork computed from the same initialisation and batches (recorded in
+    tests/golden/ref_qmix.npz by make_reference_cases)."""
+    g = load_case(LIVE, f"c{LIVE_CASES.index((tu, sharing))}")
+    it, im = _live_index(sharing)
+    n_nets = 1 if sharing else N
+    torch.manual_seed(11)   # the reference's initialisation order: agents' networks, their target copies, mixer
+    theta = lr.init_flat(n_nets, D, A)
+    lr.init_flat(n_nets, D, A)
+    mix = qr.init_mixer_flat(N, N * D, 64, 32)
+    assert np.abs(theta.numpy()[it] - g["theta0"]).max() < 1e-6 and np.abs(mix.numpy()[im] - g["mix0"]).max() < 1e-6, "initialisation differs from the reference's"
+    st = qr.QmixState(theta.clone(), theta.clone(), mix.clone(), mix.clone(), [0] * N if sharing else list(range(N)), D, A)
+    assert st.mix.numel() == qr.mixer_size(N, N * D, 64, 32) == int(g["n_mix"])
     rng = np.random.default_rng(5)
     hp = lr.DqnHP(target_update_interval_or_tau=tu)
-    for _ in range(3):
+    for want in g["loss"]:
         b = _batch(rng, 16)
-        want = model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"]
         got = qr.qmix_update(st, b, hp)
         assert abs(got["loss"] - want) <= 1e-5 * max(1.0, abs(want))
-    sd = model.state_dict()
-    for mine, theirs in ((st.theta, lr.flat_from_state_dict(sd, f"critic.{kind}", n_nets)), (st.theta_tgt, lr.flat_from_state_dict(sd, f"target.{kind}", n_nets)),
-                         (st.mix, qr.mixer_flat_from_state_dict(sd, "mixer")), (st.mix_tgt, qr.mixer_flat_from_state_dict(sd, "target_mixer"))):
-        assert np.quantile(np.abs(mine.numpy() - theirs.numpy()), 0.999) < 1e-5
+    for mine, idx, key in ((st.theta, it, "theta"), (st.theta_tgt, it, "theta_tgt"), (st.mix, im, "mix"), (st.mix_tgt, im, "mix_tgt")):
+        assert np.quantile(np.abs(mine.numpy()[idx] - g[key]), 0.999) < 1e-5, key
 
 
 def make_golden():
-    """Regenerates tests/golden/qmix_indep.npz from the live reference (build container): python -c 'import tests.test_qmix as t; t.make_golden()'"""
+    """Regenerates tests/golden/qmix_indep.npz from the live reference: MARLBASE_SRC=<marlbase checkout> python -c 'import tests.test_qmix as t; t.make_golden()'"""
     from oracle import ref_shim
 
     ref = ref_shim.load()

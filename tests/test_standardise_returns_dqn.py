@@ -1,6 +1,7 @@
-"""cfg.standardise_returns of the DQN family (marlbase/dqn/model.py:82-84,147-158; VDN 221-222,256-264): the oracle against the LIVE reference
-classes (`refsrc`, build container only) and the B200 path (marl_dqn_standardise_returns) against the oracle."""
+"""cfg.standardise_returns of the DQN family (marlbase/dqn/model.py:82-84,147-158; VDN 221-222,256-264): the oracle against recorded outputs of the
+reference classes (tests/golden/ref_standardise_returns_dqn.npz) and the B200 path (marl_dqn_standardise_returns) against the oracle."""
 import copy
+import os
 import types
 
 import numpy as np
@@ -8,6 +9,7 @@ import pytest
 import torch
 
 from oracle import learner_ref as lr
+from tests.helpers import load_case, net_layers, sample_index
 
 N, D, A, T = 2, 15, 6, 25
 
@@ -35,26 +37,50 @@ def _store(rng, cap, coop):
     return dict(obs=obs, act=act, rew=rew, done=done, filled=filled)
 
 
-@pytest.mark.refsrc
-@pytest.mark.parametrize("cls,mixer", [("QNetwork", 0), ("VDNetwork", 1)])
-def test_oracle_matches_live_reference(cls, mixer):
+LIVE = os.path.join(os.path.dirname(__file__), "golden", "ref_standardise_returns_dqn.npz")
+
+
+def _live_batches(mixer, B=12):
+    rng = np.random.default_rng(8)
+    for _ in range(3):
+        s = _store(rng, 40, bool(mixer))
+        yield lr.batch_from_store(s, rng.integers(0, 40, size=B).astype(np.int32))
+
+
+def make_reference_cases():
+    """Records tests/golden/ref_standardise_returns_dqn.npz from the reference's QNetwork / VDNetwork: MARLBASE_SRC=<marlbase checkout> python -c
+    'import tests.test_standardise_returns_dqn as t; t.make_reference_cases()'."""
     from oracle import ref_shim
 
     ref = ref_shim.load()
+    idx = sample_index(net_layers(N, D, A))
+    out = {}
+    for cls in ("QNetwork", "VDNetwork"):
+        torch.manual_seed(3)
+        model = getattr(ref.dqn_model, cls)([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, ref_shim.dqn_cfg(standardise_returns=True), [128, 128], False, False, True, "cpu")
+        out[f"{cls}.theta0"] = lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy()[idx]
+        losses = [model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"]
+                  for b in _live_batches(int(cls == "VDNetwork"))]
+        out.update({f"{cls}.loss": np.array(losses, np.float64), f"{cls}.ret_mean": model.ret_ms.mean.numpy(), f"{cls}.ret_var": model.ret_ms.var.numpy(),
+                    f"{cls}.theta": lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy()[idx]})
+    np.savez_compressed(LIVE, **out)
+
+
+@pytest.mark.parametrize("cls,mixer", [("QNetwork", 0), ("VDNetwork", 1)])
+def test_oracle_matches_live_reference(cls, mixer):
+    """Three updates of the oracle against what the reference's class computed from the same initialisation and batches (recorded by
+    make_reference_cases)."""
+    g = load_case(LIVE, cls)
+    idx = sample_index(net_layers(N, D, A))
     torch.manual_seed(3)
-    model = getattr(ref.dqn_model, cls)([ref_shim.Space(shape=(D,))] * N, [ref_shim.Space(n=A)] * N, ref_shim.dqn_cfg(standardise_returns=True), [128, 128], False, False, True, "cpu")
-    theta = lr.flat_from_state_dict(model.state_dict(), "critic.independent", N)
+    theta = lr.init_flat(N, D, A)
+    assert np.abs(theta.numpy()[idx] - g["theta0"]).max() < 1e-6, "initialisation differs from the reference's"
     st = lr.DqnState(theta.clone(), theta.clone(), [0, 1], D, A, ret_ms=lr.RunningMeanStdRef((1,) if mixer else (N,)))
     hp = lr.DqnHP(mixer=mixer)
-    rng = np.random.default_rng(8)
-    B = 12
-    for _ in range(3):
-        s = _store(rng, 40, bool(mixer))
-        b = lr.batch_from_store(s, rng.integers(0, 40, size=B).astype(np.int32))
-        want = model.update(ref.dqn_train.Batch(b["obss"], b["actions"], b["rewards"], b["dones"], b["filled"], None))["loss"]
+    for b, want in zip(_live_batches(mixer), g["loss"], strict=True):
         _close(lr.dqn_update(st, b, hp)["loss"], want)
-    _close(st.ret_ms.mean.numpy(), model.ret_ms.mean.numpy()); _close(st.ret_ms.var.numpy(), model.ret_ms.var.numpy())
-    d = np.abs(st.theta.numpy() - lr.flat_from_state_dict(model.state_dict(), "critic.independent", N).numpy())
+    _close(st.ret_ms.mean.numpy(), g["ret_mean"]); _close(st.ret_ms.var.numpy(), g["ret_var"])
+    d = np.abs(st.theta.numpy()[idx] - g["theta"])
     assert np.quantile(d, 0.999) < 1e-5
 
 
