@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from .. import _native as nat
-from ..dqn.model import HIDDEN, _dim, flat_to_state_dict, init_flat_params, sharing_to_nets, state_dict_to_flat
+from ..dqn.model import HIDDEN, _dim, check_in_dim, flat_to_state_dict, init_flat_params, sharing_to_nets, state_dict_to_flat
 from ..lbf import TrajStore
 
 
@@ -37,9 +37,8 @@ class A2CNetwork:
         # critic.centralised (MAA2C / MAPPO, ac/model.py:62-65): every agent's critic reads the concatenation of all agents' observations
         self.centralised = bool(critic.centralised) and self.n_agents > 1
         self.critic_in = self.n_agents * self.in_dim if self.centralised else self.in_dim
-        if self.critic_in > 32:
-            raise NotImplementedError(f"critic.centralised: the joint observation is {self.critic_in} wide; the learner kernels stage at most 32 input features "
-                                      "(2 agents on Foraging-8x8-2p-3f: 30)")
+        check_in_dim(self.in_dim, "the observation")
+        check_in_dim(self.critic_in, "critic.centralised: the joint observation")
         self.gamma, self.entropy_coef, self.n_steps = float(cfg.gamma), float(cfg.entropy_coef), int(cfg.n_steps)
         self.grad_clip, self.value_loss_coef = cfg.grad_clip, float(cfg.value_loss_coef)
         self.target_update_interval_or_tau = float(cfg.target_update_interval_or_tau)

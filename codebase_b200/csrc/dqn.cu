@@ -378,7 +378,7 @@ int marl_dqn_forward(marl_dqn* h, const float* obs, int32_t n_envs, int32_t use_
   src.mode = 0; src.dense = obs; src.E = n_envs; src.N = h->ns.n_agents; src.D = h->ns.in;
   bool& current = use_target ? h->tgt_image_current : h->image_current;
   const int rc = forward_any(h->ns, plan, src, use_target ? h->theta_tgt : h->theta, use_target ? h->image_tgt : h->image, q_out, (cudaStream_t)stream, current);
-  if (rc == MARL_OK) current = tc_forward_enabled() != 0;
+  if (rc == MARL_OK) current = tc_forward_for(h->ns);
   return rc;
 }
 
@@ -407,7 +407,7 @@ static int dqn_grads(marl_dqn* h, const marl_traj_view* traj, const int32_t* epi
     h->tq_ahead = false;
   } else {
     if (int rc = forward_any(h->ns, plan, src, h->theta_tgt, h->image_tgt, h->tq, st, h->tgt_image_current)) return rc;
-    h->tgt_image_current = tc_forward_enabled() != 0;
+    h->tgt_image_current = tc_forward_for(h->ns);
   }
   int n_loss_parts = plan.cta_begin[plan.n_nets];
   const float* td_ext = nullptr;
@@ -418,7 +418,7 @@ static int dqn_grads(marl_dqn* h, const marl_traj_view* traj, const int32_t* epi
     MARL_REQUIRE(h->hp.mixer == 0 || batch == h->n_stat, "marl_dqn_update: VDN's standardise_returns keeps one statistic per batch entry (the reference's reshape(-1, B)): "
                  "batch %d must stay at max_batch %d", batch, h->n_stat);
     if (int rc = forward_any(h->ns, plan, src, h->theta, h->image, h->q_all, st, h->image_current)) return rc;
-    h->image_current = tc_forward_enabled() != 0;
+    h->image_current = tc_forward_for(h->ns);
     const int C = h->hp.mixer == 1 ? 1 : h->ns.n_agents;
     StdRetParams sp; memset(&sp, 0, sizeof(sp));
     sp.q = h->q_all; sp.tq = h->tq; sp.traj = src.traj; sp.idx = episode_idx; sp.B = batch; sp.N = h->ns.n_agents; sp.A = h->ns.out; sp.vdn = h->hp.mixer == 1;
@@ -437,7 +437,7 @@ static int dqn_grads(marl_dqn* h, const marl_traj_view* traj, const int32_t* epi
     td_agent_stride = h->hp.mixer == 1 ? 0 : batch * T;
   } else if (h->hp.mixer == 1) {  // VDN: online Q-values of all agents first, then the agent-summed TD error
     if (int rc = forward_any(h->ns, plan, src, h->theta, h->image, h->q_all, st, h->image_current)) return rc;
-    h->image_current = tc_forward_enabled() != 0;
+    h->image_current = tc_forward_for(h->ns);
     VdnTdParams vp; vp.q = h->q_all; vp.tq = h->tq; vp.traj = src.traj; vp.idx = episode_idx; vp.B = batch; vp.N = h->ns.n_agents; vp.A = h->ns.out;
     vp.gamma = h->hp.gamma; vp.double_q = h->hp.double_q; vp.td = h->td;
     const int vb = (batch * T + 255) / 256;
@@ -449,7 +449,7 @@ static int dqn_grads(marl_dqn* h, const marl_traj_view* traj, const int32_t* epi
   } else if (h->hp.mixer == 2) {  // QMIX: the mixer turns the agents' Q-values into the TD error and hands dL/dq_a back per agent (qmix.cuh)
     MARL_REQUIRE(h->mix != nullptr, "marl_dqn_update: QMIX needs marl_dqn_qmix_init first");
     if (int rc = forward_any(h->ns, plan, src, h->theta, h->image, h->q_all, st, h->image_current)) return rc;
-    h->image_current = tc_forward_enabled() != 0;
+    h->image_current = tc_forward_for(h->ns);
     QmixParams qp; memset(&qp, 0, sizeof(qp));
     qp.L = h->ql; qp.q = h->q_all; qp.tq = h->tq; qp.traj = src.traj; qp.idx = episode_idx; qp.B = batch; qp.A = h->ns.out; qp.D = h->ns.in;
     qp.gamma = h->hp.gamma; qp.double_q = h->hp.double_q; qp.mix = h->mix; qp.mix_tgt = h->mix_tgt; qp.rec = h->mix_rec; qp.td = h->td;
@@ -476,12 +476,12 @@ static int dqn_grads(marl_dqn* h, const marl_traj_view* traj, const int32_t* epi
   tp.gamma = h->hp.gamma; tp.double_q = h->hp.double_q; tp.scratch = h->scratch; tp.scratch_pitch = h->scratch_pitch; tp.loss_part = loss_part;
   const bool rec = h->timing && h->ev_used < kTimingPairs;
   if (rec) cudaEventRecord(h->ev[4 * h->ev_used], st);
-  if (tc_backward_enabled() && h->ns.in < kMaxObsDim) {
+  if (tc_backward_enabled() && h->ns.in < kTcObsDim) {
     if (!h->tc_h1) {  // intermediates of the tensor-core pipeline, allocated on first use
       const size_t rows = (size_t)h->ns.n_agents * h->max_batch * (h->max_T + 1);
       int rc = 0;
       rc |= dqn_alloc(&h->tc_h1, rows * kHidden); rc |= dqn_alloc(&h->tc_h2, rows * kHidden);
-      rc |= dqn_alloc(&h->tc_dh1, rows * kHidden); rc |= dqn_alloc(&h->tc_rec, rows * 16 /* kRowRec */); rc |= dqn_alloc(&h->tc_x, rows * kMaxObsDim);
+      rc |= dqn_alloc(&h->tc_dh1, rows * kHidden); rc |= dqn_alloc(&h->tc_rec, rows * 16 /* kRowRec */); rc |= dqn_alloc(&h->tc_x, rows * kTcObsDim);
       rc |= dqn_alloc(reinterpret_cast<float**>(&h->image_bwd), (size_t)h->ns.n_nets * tc_bwd_image_bytes() / 4 + 4);
       if (rc) return MARL_ENOMEM;
     }
@@ -523,7 +523,7 @@ static void dqn_adam_params(marl_dqn* h, float* loss_out, AdamParams& ap) {
   ap.loss_out = loss_out ? loss_out : h->loss_dev;
   ap.sumsq_part = h->grads_are_local ? h->sumsq : nullptr; ap.n_sumsq = (int)((h->n_params + 63) / 64);
   h->grads_are_local = false;
-  if (h->image != nullptr && tc_forward_enabled()) {  // valid images stay valid: adam_kernel rewrites the entries of every parameter it steps
+  if (h->image != nullptr && tc_forward_for(h->ns)) {  // valid images stay valid: adam_kernel rewrites the entries of every parameter it steps (a wide network has none)
     ap.image = h->image; ap.bwd_image = h->image_bwd; ap.img_lay = h->ns.lay; ap.img_nets = h->ns.n_nets;
     ap.image_bytes = tc_image_bytes(); ap.bwd_image_bytes = tc_bwd_image_bytes();
     if (h->image_bwd == nullptr) h->bwd_image_current = false;
@@ -576,7 +576,7 @@ static int dqn_update(marl_dqn* h, const marl_traj_view* traj, const int32_t* ep
         RowSource src; memset(&src, 0, sizeof(src));
         src.mode = 1; src.traj = to_view(traj); src.idx = next->idx; src.N = h->ns.n_agents; src.D = h->ns.in;
         if (int rc = forward_any(h->ns, plan, src, h->theta_tgt, h->image_tgt, h->tq, (cudaStream_t)stream, h->tgt_image_current)) return rc;
-        h->tgt_image_current = tc_forward_enabled() != 0;
+        h->tgt_image_current = tc_forward_for(h->ns);
         h->tq_ahead = true;
       }
       if (int rc = launch_adam_finish(rp, ap, &h->xchg, h->grid_barrier, &h->grid_epoch, h->n_sm, (cudaStream_t)stream)) return rc;

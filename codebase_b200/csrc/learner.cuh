@@ -6,7 +6,8 @@
 
 namespace marl {
 
-constexpr int kMaxObsDim = 32;  // KP = 16 or 32 float input tiles
+constexpr int kMaxObsDim = 128;  // FP32 FFMA kernels: KP = 16 or 32 float input tiles, KP = kKpWide (K-chunked layer 1) above 32
+constexpr int kTcObsDim = 32;    // tensor-core kernels: the staged input width (one 32-feature W1 panel, the `xg` row pitch); wider networks use FFMA
 
 struct TrajView {  // device view of marl_traj_view
   const float* obs; const int32_t* act; const float* rew; const uint8_t* done; const uint8_t* filled;
@@ -99,15 +100,28 @@ __device__ __forceinline__ void setup_rows(RowMeta* m, const RowPlan& p, const R
 }
 
 // Fill the [128][KP] input tile from the staged row pointers (asynchronous copies; zero padding in both directions).
+// KP = kKpWide: only the ceil(D / kW1Chunk) * kW1Chunk leading columns the K-chunks read, one row per warp and pass.
 // Caller: cp_async_wait_all() + __syncthreads() before the tile is read.
 template <int KP>
 __device__ __forceinline__ void gather_tile_async(float* X, const RowMeta* m, int D) {
+  if constexpr (KP == kKpWide) {
+    const int cols = (D + kW1Chunk - 1) / kW1Chunk * kW1Chunk, lane = threadIdx.x & 31;
+#pragma unroll 2
+    for (int r = threadIdx.x >> 5; r < kTileRows; r += kMlpThreads / 32) {
+      const float* src = m->src[r];
+      for (int k = lane; k < cols; k += 32) {
+        if (src != nullptr && k < D) cp_async4(&at1<KP>(X, r, k), src + k);
+        else at1<KP>(X, r, k) = 0.f;
+      }
+    }
+  } else {
 #pragma unroll 4
-  for (int i = threadIdx.x; i < kTileRows * KP; i += kMlpThreads) {
-    const int r = i / KP, k = i - r * KP;
-    const float* src = m->src[r];
-    if (src != nullptr && k < D) cp_async4(&at1<KP>(X, r, k), src + k);
-    else at1<KP>(X, r, k) = 0.f;
+    for (int i = threadIdx.x; i < kTileRows * KP; i += kMlpThreads) {
+      const int r = i / KP, k = i - r * KP;
+      const float* src = m->src[r];
+      if (src != nullptr && k < D) cp_async4(&at1<KP>(X, r, k), src + k);
+      else at1<KP>(X, r, k) = 0.f;
+    }
   }
 }
 
@@ -262,18 +276,21 @@ struct TcBuffers {
   uint8_t* image; uint8_t* bwd_image;       // packed online-network images (forward K-major, backward K-major W2^T)
   float *h1, *h2, *dh1;                     // [32][rows][4] (chunk-major) activations and hidden-layer gradient
   float* rec;                               // [rows][16] row records (tc_train.cu)
-  float* x;                                 // [rows][kMaxObsDim] gathered observation rows
+  float* x;                                 // [rows][kTcObsDim] gathered observation rows
   size_t rows;                              // allocated rows
 };
 int tc_train_init();
 int launch_tc_dqn_train(const TrainParams& tp, const TcBuffers& buf, cudaStream_t st, cudaEvent_t* between = nullptr);  // between[2]: recorded after kernels 1 and 2
 // tc_forward_enabled(): process-wide switch (marl_set_option("tensor_core_forward", 0|1)), declared in common.cuh
+// Does a forward of this network set run on the tensor cores?  Only up to kTcObsDim inputs: a wider network (a MAPPO learner's centralised
+// critic next to its narrow actor, say) always takes the FFMA kernels, and no packed image is ever built or kept for it.
+inline bool tc_forward_for(const NetSet& ns) { return tc_forward_enabled() && ns.in <= kTcObsDim; }
 
 // Forward pass through whichever implementation is selected.  `image` is scratch for the packed weights (n_nets images);
 // it is rebuilt from `theta` on every call (3 us) so that it can never go stale against direct parameter writes.
 inline int forward_any(const NetSet& ns, const RowPlan& plan, const RowSource& src, const float* theta, uint8_t* image, float* out, cudaStream_t st,
                        bool image_is_current = false) {
-  if (tc_forward_enabled() && image != nullptr) {
+  if (tc_forward_for(ns) && image != nullptr) {
     if (!image_is_current)
       if (int rc = launch_pack_weights(theta, ns.lay, ns.n_nets, image, st)) return rc;
     FwdParams fp; fp.plan = plan; fp.src = src; fp.theta = theta; fp.lay = ns.lay; fp.out = out;

@@ -29,16 +29,19 @@ __global__ void __launch_bounds__(kMlpThreads, 1) mlp_forward_kernel(FwdParams p
   int net, row_begin, row_end;
   cta_rows(p.plan, net, row_begin, row_end);
   if (row_begin >= row_end) return;
-  w.load_async(p.theta + (size_t)net * p.lay.P, p.lay);
+  const float* theta = p.theta + (size_t)net * p.lay.P;
+  w.load_async(theta, p.lay);
   for (int vr0 = row_begin; vr0 < row_end; vr0 += kTileRows) {
     const int nrows = min(kTileRows, row_end - vr0);
     __syncthreads();
     setup_rows<false>(meta, p.plan, p.src, net, vr0, nrows);
     __syncthreads();
     gather_tile_async<KP>(X, meta, p.src.D);
+    if constexpr (KP == kKpWide) w.load_w1_chunk_async(theta, p.lay, 0);
     cp_async_wait_all();
     __syncthreads();
-    mlp_forward_tile<KP>(X, H1, H2, Q, w, tc);
+    if constexpr (KP == kKpWide) mlp_forward_tile_wide(X, H1, H2, Q, w, theta, p.lay, tc);
+    else mlp_forward_tile<KP>(X, H1, H2, Q, w, tc);
     __syncthreads();
     for (int i = threadIdx.x; i < nrows * p.lay.out; i += kMlpThreads) {
       const int r = i / p.lay.out, o = i - r * p.lay.out;
@@ -180,7 +183,37 @@ __device__ __forceinline__ void mlp_backward_tile(float* X, float* H1, float* H2
   cp_async_wait_all();
   __syncthreads();
   // ---- dW1[m][i] = sum_r dh1[r][m] * x[r][i] ---------------------------------------------------------------------
-  {
+  if constexpr (KP == kKpWide) {
+    // one pass per K-chunk of the input (the narrow tiles' two-column-group register block), dH1 re-read from shared memory per pass:
+    // a single 128-column pass would hold 64 more accumulators than the register budget has
+    const int mg = t >> 4, i0 = t & 15, n_chunks = (lay.in + kW1Chunk - 1) / kW1Chunk;
+#pragma unroll 1
+    for (int c = 0; c < n_chunks; ++c) {
+      float acc[kW1Chunk / 16][8];
+#pragma unroll
+      for (int ii = 0; ii < kW1Chunk / 16; ++ii)
+#pragma unroll
+        for (int q = 0; q < 8; ++q) acc[ii][q] = 0.f;
+#pragma unroll 4
+      for (int r = 0; r < kTileRows; ++r) {
+        const float4 a0 = at4<kHidden>(H1, r, 2 * mg), a1 = at4<kHidden>(H1, r, 2 * mg + 1);
+#pragma unroll
+        for (int ii = 0; ii < kW1Chunk / 16; ++ii) {
+          const float x = at1<KP>(X, r, c * kW1Chunk + i0 + 16 * ii);
+          acc[ii][0] = fmaf(a0.x, x, acc[ii][0]); acc[ii][1] = fmaf(a0.y, x, acc[ii][1]); acc[ii][2] = fmaf(a0.z, x, acc[ii][2]); acc[ii][3] = fmaf(a0.w, x, acc[ii][3]);
+          acc[ii][4] = fmaf(a1.x, x, acc[ii][4]); acc[ii][5] = fmaf(a1.y, x, acc[ii][5]); acc[ii][6] = fmaf(a1.z, x, acc[ii][6]); acc[ii][7] = fmaf(a1.w, x, acc[ii][7]);
+        }
+      }
+#pragma unroll
+      for (int ii = 0; ii < kW1Chunk / 16; ++ii) {
+        const int i = c * kW1Chunk + i0 + 16 * ii;
+        if (i < lay.in) {
+#pragma unroll
+          for (int q = 0; q < 8; ++q) rmw(gs + lay.w1 + (mg * 8 + q) * lay.in + i, acc[ii][q], first);
+        }
+      }
+    }
+  } else {
     const int mg = t >> 4, i0 = t & 15;
     float acc[KP / 16][8];
 #pragma unroll
@@ -310,7 +343,8 @@ __global__ void __launch_bounds__(kMlpThreads, 1) train_kernel(TrainParams p) {
     if (t < 4) p.loss_part[4 * blockIdx.x + t] = 0.f;
     return;
   }
-  w.load_async(p.theta + (size_t)net * p.lay.P, p.lay);
+  const float* theta = p.theta + (size_t)net * p.lay.P;
+  w.load_async(theta, p.lay);
   RowCtx c; c.T = p.src.traj.T; c.A = p.lay.out; c.B = p.plan.units_per_agent;
   bool first = true;
   // tiles from the top of the chunk downwards, so that the next row's outputs of a tile's last row are already known
@@ -320,9 +354,11 @@ __global__ void __launch_bounds__(kMlpThreads, 1) train_kernel(TrainParams p) {
     setup_rows<true>(meta, p.plan, p.src, net, vr0, nrows);
     __syncthreads();
     gather_tile_async<KP>(X, meta, p.src.D);
+    if constexpr (KP == kKpWide) w.load_w1_chunk_async(theta, p.lay, 0);   // (the backward never reads W1: the slot is free)
     cp_async_wait_all();
     __syncthreads();
-    mlp_forward_tile<KP>(X, H1, H2, Q, w, tc);
+    if constexpr (KP == kKpWide) mlp_forward_tile_wide(X, H1, H2, Q, w, theta, p.lay, tc);
+    else mlp_forward_tile<KP>(X, H1, H2, Q, w, tc);
     __syncthreads();
     float dq[kOutPad];
 #pragma unroll
@@ -717,13 +753,14 @@ static int init_kp() {
 
 int learner_kernels_init(int in_dim) {
   MARL_REQUIRE(in_dim >= 1 && in_dim <= kMaxObsDim, "learner kernels: observation width %d not supported (1..%d)", in_dim, kMaxObsDim);
-  return in_dim <= 16 ? init_kp<16>() : init_kp<32>();
+  return in_dim <= 16 ? init_kp<16>() : in_dim <= 32 ? init_kp<32>() : init_kp<kKpWide>();
 }
 
 int launch_mlp_forward(const FwdParams& p, cudaStream_t st) {
   const int grid = p.plan.cta_begin[p.plan.n_nets];
   if (p.lay.in <= 16) mlp_forward_kernel<16><<<grid, kMlpThreads, forward_smem_bytes<16>(), st>>>(p);
-  else mlp_forward_kernel<32><<<grid, kMlpThreads, forward_smem_bytes<32>(), st>>>(p);
+  else if (p.lay.in <= 32) mlp_forward_kernel<32><<<grid, kMlpThreads, forward_smem_bytes<32>(), st>>>(p);
+  else mlp_forward_kernel<kKpWide><<<grid, kMlpThreads, forward_smem_bytes<kKpWide>(), st>>>(p);
   MARL_CUDA_TRY(cudaGetLastError());
   return MARL_OK;
 }
@@ -741,7 +778,7 @@ static int launch_train_kp(const TrainParams& p, int head, cudaStream_t st) {
 }
 
 int launch_train(const TrainParams& p, int head, cudaStream_t st) {
-  return p.lay.in <= 16 ? launch_train_kp<16>(p, head, st) : launch_train_kp<32>(p, head, st);
+  return p.lay.in <= 16 ? launch_train_kp<16>(p, head, st) : p.lay.in <= 32 ? launch_train_kp<32>(p, head, st) : launch_train_kp<kKpWide>(p, head, st);
 }
 
 int launch_grad_reduce(const ReduceParams& p, cudaStream_t st) {

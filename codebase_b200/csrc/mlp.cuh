@@ -38,6 +38,14 @@ template <int KP>
 constexpr int pitch_of() { return KP == 128 ? 132 : KP; }
 constexpr int kPitchH = 132;
 
+// Wide inputs (33..128 features, KP = kKpWide): the input tile is gathered at full width into the H2 region ([128][132], like H2), but a
+// resident [128][128] first-layer weight tile does not fit next to W2, H1 and H2.  Layer 1 therefore walks the input in K-chunks of
+// kW1Chunk columns, staging chunk c of W1 into the [128][kW1Chunk] slot the narrow tiles keep W1 in (see mlp_forward_tile_wide).
+constexpr int kKpWide = 128;
+constexpr int kW1Chunk = 32;
+template <int KP>
+constexpr int w1_kp() { return KP == kKpWide ? kW1Chunk : KP; }   // width of the shared-memory W1 slot
+
 // physical 16-byte chunk of logical chunk c in `row`
 template <int KP>
 __device__ __forceinline__ int swz(int row, int c) {
@@ -187,21 +195,24 @@ struct NetLayout {
   }
 };
 
-// Shared-memory weight block of one network.
+// Shared-memory weight block of one network.  KP = kKpWide: the W1 slot holds one [128][kW1Chunk] K-chunk at a time (load_w1_chunk_async).
 template <int KP>
 struct WeightSmem {
-  static constexpr int kFloats = kHidden * pitch_of<KP>() + kHidden * kPitchH + kOutPad * kHidden + kHidden + kHidden + kOutPad;
+  static constexpr int kFloats = kHidden * pitch_of<w1_kp<KP>()>() + kHidden * kPitchH + kOutPad * kHidden + kHidden + kHidden + kOutPad;
   float* w1; float* w2; float* w3; float* b1; float* b2; float* b3;
   __device__ explicit WeightSmem(float* base) {
-    w1 = base; w2 = w1 + kHidden * pitch_of<KP>(); w3 = w2 + kHidden * kPitchH; b1 = w3 + kOutPad * kHidden; b2 = b1 + kHidden; b3 = b2 + kHidden;
+    w1 = base; w2 = w1 + kHidden * pitch_of<w1_kp<KP>()>(); w3 = w2 + kHidden * kPitchH; b1 = w3 + kOutPad * kHidden; b2 = b1 + kHidden; b3 = b2 + kHidden;
   }
   // cooperative asynchronous load from global params (native layouts) into the swizzled smem layouts; 4-byte
   // cp.async because theta + net*P is only 4-byte aligned.  Caller: cp_async_wait_all() + __syncthreads() before use.
+  // (KP = kKpWide: everything but W1, whose chunks are staged per tile)
   __device__ void load_async(const float* __restrict__ theta, const NetLayout& l) {
-    for (int i = threadIdx.x; i < kHidden * KP; i += kMlpThreads) {
-      const int n = i / KP, k = i % KP;
-      if (k < l.in) cp_async4(&at1<KP>(w1, n, k), theta + l.w1 + n * l.in + k);
-      else at1<KP>(w1, n, k) = 0.f;
+    if constexpr (KP != kKpWide) {
+      for (int i = threadIdx.x; i < kHidden * KP; i += kMlpThreads) {
+        const int n = i / KP, k = i % KP;
+        if (k < l.in) cp_async4(&at1<KP>(w1, n, k), theta + l.w1 + n * l.in + k);
+        else at1<KP>(w1, n, k) = 0.f;
+      }
     }
 #pragma unroll 8
     for (int i = threadIdx.x; i < kHidden * kHidden; i += kMlpThreads) cp_async4(&at1<kHidden>(w2, i / kHidden, i % kHidden), theta + l.w2 + i);
@@ -212,7 +223,41 @@ struct WeightSmem {
     for (int i = threadIdx.x; i < kHidden; i += kMlpThreads) { cp_async4(b1 + i, theta + l.b1 + i); cp_async4(b2 + i, theta + l.b2 + i); }
     if (threadIdx.x < kOutPad) b3[threadIdx.x] = threadIdx.x < l.out ? theta[l.b3 + threadIdx.x] : 0.f;
   }
+  // KP = kKpWide: W1[:, c*kW1Chunk .. +kW1Chunk) into the W1 slot (columns >= in zeroed); one warp reads 32 consecutive floats of a row.
+  // Caller: the slot's previous readers are past a barrier; cp_async_wait_all() + __syncthreads() before use.
+  __device__ void load_w1_chunk_async(const float* __restrict__ theta, const NetLayout& l, int c) const {
+    const int k0 = c * kW1Chunk;
+#pragma unroll 4
+    for (int i = threadIdx.x; i < kHidden * kW1Chunk; i += kMlpThreads) {
+      const int n = i / kW1Chunk, k = i % kW1Chunk;
+      if (k0 + k < l.in) cp_async4(&at1<kW1Chunk>(w1, n, k), theta + l.w1 + n * l.in + k0 + k);
+      else at1<kW1Chunk>(w1, n, k) = 0.f;
+    }
+  }
 };
+
+// ---- NT over one K-chunk of a wide input: acc[i][j] += sum_{k < kW1Chunk} X[r_i][c*kW1Chunk + k] * W1c[n_j][k] ------------------------
+// X: the full-width [128][132] input tile, W1c: the staged [128][kW1Chunk] chunk (same thread mapping as gemm_nt)
+__device__ __forceinline__ void gemm_nt_chunk(const float* __restrict__ X, int c, const float* __restrict__ W1c, const ThreadCoord& tc, float (&acc)[8][8]) {
+  const int r0 = tc.wy * 32 + tc.ty, n0 = tc.wx * 64 + tc.tx, q0 = c * (kW1Chunk / 4);
+#pragma unroll 2
+  for (int q = 0; q < kW1Chunk / 4; ++q) {
+    float4 a[8], b[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) a[i] = at4<kKpWide>(X, r0 + 4 * i, q0 + q);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) b[j] = at4<kW1Chunk>(W1c, n0 + 8 * j, q);
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        acc[i][j] = fmaf(a[i].x, b[j].x, acc[i][j]);
+        acc[i][j] = fmaf(a[i].y, b[j].y, acc[i][j]);
+        acc[i][j] = fmaf(a[i].z, b[j].z, acc[i][j]);
+        acc[i][j] = fmaf(a[i].w, b[j].w, acc[i][j]);
+      }
+  }
+}
 
 // x -> h1 -> h2 -> q for one 128-row tile (all buffers in shared memory; caller syncs before use of q).
 template <int KP>
@@ -220,6 +265,33 @@ __device__ __forceinline__ void mlp_forward_tile(const float* X, float* H1, floa
   float acc[8][8];
   zero_acc(acc);
   gemm_nt<KP>(X, w.w1, tc, acc);
+  store_relu_bias(H1, w.b1, tc, acc);
+  __syncthreads();
+  zero_acc(acc);
+  gemm_nt<kHidden>(H1, w.w2, tc, acc);
+  store_relu_bias(H2, w.b2, tc, acc);
+  __syncthreads();
+  head_forward(H2, w.w3, w.b3, Q);
+}
+
+// The same for a wide input (KP = kKpWide).  On entry X holds the tile's ceil(in / kW1Chunk) * kW1Chunk leading columns and the W1 slot
+// holds chunk 0 (staged with the tile, waited for and synced by the caller).  Chunks 1.. are staged here from `theta` (this network's
+// parameters, L2-resident), each after every thread is done with the previous one, into the same accumulators: layer 1 costs
+// ceil(in / 32) chunk round trips per tile instead of holding a [128][128] W1 that does not fit next to W2, H1 and H2.
+__device__ __forceinline__ void mlp_forward_tile_wide(const float* X, float* H1, float* H2, float* Q, const WeightSmem<kKpWide>& w, const float* theta,
+                                                      const NetLayout& lay, const ThreadCoord& tc) {
+  const int n_chunks = (lay.in + kW1Chunk - 1) / kW1Chunk;
+  float acc[8][8];
+  zero_acc(acc);
+  gemm_nt_chunk(X, 0, w.w1, tc, acc);
+#pragma unroll 1
+  for (int c = 1; c < n_chunks; ++c) {
+    __syncthreads();   // every thread is done with chunk c - 1
+    w.load_w1_chunk_async(theta, lay, c);
+    cp_async_wait_all();
+    __syncthreads();
+    gemm_nt_chunk(X, c, w.w1, tc, acc);
+  }
   store_relu_bias(H1, w.b1, tc, acc);
   __syncthreads();
   zero_acc(acc);

@@ -259,7 +259,7 @@ struct TcTrainParams {
   // reads 512 contiguous bytes per instruction (row-major rows of 512 B cost one cache line per lane and instruction)
   float* h1g; float* h2g; float* dh1g; size_t rows;
   float* rec;                 // [rows][kRowRec] row records
-  float* xg;                  // [rows][kMaxObsDim] gathered observation rows (zero padded to the staged width): the weight-gradient
+  float* xg;                  // [rows][kTcObsDim] gathered observation rows (zero padded to the staged width): the weight-gradient
                               // kernel reads them without chasing the episode index again
   const float* tq; const float* td_ext; int td_agent_stride; float gamma; int double_q;
   float* scratch; int scratch_pitch; float* loss_part;
@@ -295,7 +295,7 @@ __device__ __forceinline__ void issue_l1_ss(uint32_t d_tmem, uint32_t xs_hi, uin
 #pragma unroll
   for (int term = 0; term < 3; ++term)
 #pragma unroll
-    for (int ks = 0; ks < kMaxObsDim / 8; ++ks)
+    for (int ks = 0; ks < kTcObsDim / 8; ++ks)
       if (ks < ksteps) mma_tf32_ss(d_tmem, (term == 0 ? alo : ahi) + (uint32_t)((ks * 32) >> 4), (term == 1 ? blo : bhi) + (uint32_t)((ks * 32) >> 4), idesc, (term | ks) ? 1u : 0u);
 }
 // this thread's 8 observation columns of its row -> the K-major SWIZZLE_128B X tile (hi | lo): 16-byte chunk c of row r sits at chunk c ^ (r & 7)

@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) tc_forward_kernel(FwdParams p, 
     // ---- layer 1 -------------------------------------------------------------------------------------------------
     if (t == 0) {
       tc_fence_after();
-      issue_layer<kMaxObsDim / 8, kHidden, kPanelBytes>(tmem, d_cur, smem_base + kOffW1Hi, smem_base + kOffW1Lo, k1steps);
+      issue_layer<kTcObsDim / 8, kHidden, kPanelBytes>(tmem, d_cur, smem_base + kOffW1Hi, smem_base + kOffW1Lo, k1steps);
       mma_commit(bar);
     }
     mbar_wait(bar, parity); parity ^= 1;
@@ -356,7 +356,7 @@ __global__ void __launch_bounds__(kP2Threads, 1) tc_forward2_kernel(FwdParams p,
       const int rem = vr - rs[m].slot * rpa;
       rs[m].unit = rem / urows; rs[m].off = rem - rs[m].unit * urows;
     }
-    float xv[2][kMaxObsDim];
+    float xv[2][kTcObsDim];
     uint32_t dst[2];
     auto fetch = [&](int tile) {   // registers <- this thread's rows of `tile` (loads stay in flight until they are staged); advances the row state
 #pragma unroll
@@ -364,7 +364,7 @@ __global__ void __launch_bounds__(kP2Threads, 1) tc_forward2_kernel(FwdParams p,
         const int row = i + m * kP2Loaders;
         dst[m] = 0xFFFFFFFFu;
 #pragma unroll
-        for (int j = 0; j < kMaxObsDim; ++j) xv[m][j] = 0.f;
+        for (int j = 0; j < kTcObsDim; ++j) xv[m][j] = 0.f;
         if (row < kTileRows && row_begin + tile * kTileRows + row < row_end && rs[m].slot < n_slots) {
           const int agent = p.plan.slot_agent[p.plan.slot_begin[net] + rs[m].slot];
           const TrajView& tv = p.src.traj;
@@ -375,7 +375,7 @@ __global__ void __launch_bounds__(kP2Threads, 1) tc_forward2_kernel(FwdParams p,
             dst[m] = (uint32_t)(((size_t)agent * rpa_units + rs[m].unit) * urows + rs[m].off);
           }
 #pragma unroll
-          for (int j = 0; j < kMaxObsDim; ++j) if (j < D) xv[m][j] = src[j];
+          for (int j = 0; j < kTcObsDim; ++j) if (j < D) xv[m][j] = src[j];
         }
         // next tile: + 128 rows
         rs[m].off += r128; rs[m].unit += q128;
@@ -390,7 +390,7 @@ __global__ void __launch_bounds__(kP2Threads, 1) tc_forward2_kernel(FwdParams p,
         if (row < kTileRows) {
           float x8[8];
 #pragma unroll
-          for (int ch = 0; ch < kMaxObsDim / 8; ++ch) {
+          for (int ch = 0; ch < kTcObsDim / 8; ++ch) {
             if (ch < k1steps) {
 #pragma unroll
               for (int j = 0; j < 8; ++j) x8[j] = xv[m][8 * ch + j];

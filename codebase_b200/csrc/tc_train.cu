@@ -153,7 +153,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) tc_dqn_fwd_kernel(TcTrainParams
       tmem_st8(lane_base + kColAHi + 8 * cq, hi);
       tmem_st8(lane_base + kColALo + 8 * cq, lo);
       if (r < nrows) {
-        float4* xo = reinterpret_cast<float4*>(p.xg + cur.dst * kMaxObsDim + 8 * cq);
+        float4* xo = reinterpret_cast<float4*>(p.xg + cur.dst * kTcObsDim + 8 * cq);
         xo[0] = make_float4(cur.x[0], cur.x[1], cur.x[2], cur.x[3]); xo[1] = make_float4(cur.x[4], cur.x[5], cur.x[6], cur.x[7]);
       }
     }
@@ -164,7 +164,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) tc_dqn_fwd_kernel(TcTrainParams
     TSG(g_ts_fwd, 3 + 6 * ts_tile);
     if (t == 0) {
       tc_fence_after();
-      issue_kmajor<kMaxObsDim / 8, kHidden, kPanelBytes>(tmem, kColD, smem_base + kOffW1Hi, smem_base + kOffW1Lo, k1steps);
+      issue_kmajor<kTcObsDim / 8, kHidden, kPanelBytes>(tmem, kColD, smem_base + kOffW1Hi, smem_base + kOffW1Lo, k1steps);
       mma_commit(bar);
       if (vr_hi != row_end) {   // every thread is past the previous tile's TD head: publish its first row's outputs
 #pragma unroll
@@ -567,7 +567,7 @@ __global__ void __launch_bounds__(kDwThreads, 1) tc_dw_kernel(TcTrainParams p) {
         pre.h1 = reinterpret_cast<const float4*>(p.h1g)[hi];
         pre.dh1 = reinterpret_cast<const float4*>(p.dh1g)[hi];
         pre.h2 = reinterpret_cast<const float4*>(p.h2g)[hi];
-        pre.xv = c4 < D ? p.xg[d * kMaxObsDim + c4] : (c4 == D ? 1.f : 0.f);   // [X | 1]: the ones column carries db1
+        pre.xv = c4 < D ? p.xg[d * kTcObsDim + c4] : (c4 == D ? 1.f : 0.f);   // [X | 1]: the ones column carries db1
       }
     };
     auto stage = [&](uint8_t* bufp, const Pre& pre) {
@@ -734,7 +734,7 @@ int tc_train_init() {
 
 // all three kernels walk the same episode-aligned row split, so the per-CTA partials line up with ReduceParams::cta_begin
 int launch_tc_dqn_train(const TrainParams& tp, const TcBuffers& buf, cudaStream_t st, cudaEvent_t* between) {
-  MARL_REQUIRE(tp.lay.in < kMaxObsDim, "tensor-core backward: observation width %d needs a spare column for the bias trick (max %d)", tp.lay.in, kMaxObsDim - 1);
+  MARL_REQUIRE(tp.lay.in < kTcObsDim, "tensor-core backward: observation width %d needs a spare column for the bias trick (max %d)", tp.lay.in, kTcObsDim - 1);
   TcTrainParams p; memset(&p, 0, sizeof(p));
   p.plan = tp.plan; p.src = tp.src; p.lay = tp.lay; p.images = buf.image; p.bwd_images = buf.bwd_image; p.q_out = nullptr;
   p.h1g = buf.h1; p.h2g = buf.h2; p.dh1g = buf.dh1; p.rec = buf.rec; p.xg = buf.x; p.rows = buf.rows;

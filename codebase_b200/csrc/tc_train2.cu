@@ -114,7 +114,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) tc_dqn_fwd2_kernel(TcTrainParam
       const int rem = vrc - rs[m].slot * rpa;
       rs[m].unit = rem / urows; rs[m].off = rem - rs[m].unit * urows;
     }
-    float xv[2][kMaxObsDim];
+    float xv[2][kTcObsDim];
     RowMeta4 mt[2];
     auto fetch = [&](int tile) {
 #pragma unroll
@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) tc_dqn_fwd2_kernel(TcTrainParam
         const int row = i + m * kT2Loaders;
         mt[m].dst = 0xFFFFFFFFu; mt[m].act_flags = 0; mt[m].rew = 0.f; mt[m].td = 0.f;
 #pragma unroll
-        for (int j = 0; j < kMaxObsDim; ++j) xv[m][j] = 0.f;
+        for (int j = 0; j < kTcObsDim; ++j) xv[m][j] = 0.f;
         const int vr = row_end - (tile + 1) * kTileRows + row;
         if (row < kTileRows && vr >= row_begin) {
           const int agent = p.plan.slot_agent[p.plan.slot_begin[net] + rs[m].slot], b = rs[m].unit, tt = rs[m].off;
@@ -131,7 +131,7 @@ __global__ void __launch_bounds__(kT2Threads, 1) tc_dqn_fwd2_kernel(TcTrainParam
           const float* src = tv.obs + ((ep * tv.N + agent) * (size_t)(T + 1) + tt) * D;
           mt[m].dst = (uint32_t)(((size_t)agent * B + b) * urows + tt);
 #pragma unroll
-          for (int j = 0; j < kMaxObsDim; ++j) if (j < D) xv[m][j] = src[j];
+          for (int j = 0; j < kTcObsDim; ++j) if (j < D) xv[m][j] = src[j];
           uint32_t fl = 0u;
           if (tt < T) {
             const uint32_t act = (uint32_t)tv.act[(ep * tv.N + agent) * T + tt];
@@ -155,13 +155,13 @@ __global__ void __launch_bounds__(kT2Threads, 1) tc_dqn_fwd2_kernel(TcTrainParam
         if (row < kTileRows) {
           float x8[8];
 #pragma unroll
-          for (int ch = 0; ch < kMaxObsDim / 8; ++ch) {
+          for (int ch = 0; ch < kTcObsDim / 8; ++ch) {
             if (ch < k1steps) {
 #pragma unroll
               for (int j = 0; j < 8; ++j) x8[j] = xv[m][8 * ch + j];
               stage_x_tile(xs, row, ch, x8);
               if (mt[m].dst != 0xFFFFFFFFu) {   // the weight-gradient kernel reads the gathered row instead of chasing the episode index again
-                float4* xo = reinterpret_cast<float4*>(p.xg + (size_t)mt[m].dst * kMaxObsDim + 8 * ch);
+                float4* xo = reinterpret_cast<float4*>(p.xg + (size_t)mt[m].dst * kTcObsDim + 8 * ch);
                 xo[0] = make_float4(x8[0], x8[1], x8[2], x8[3]); xo[1] = make_float4(x8[4], x8[5], x8[6], x8[7]);
               }
             }

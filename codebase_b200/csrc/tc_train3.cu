@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) tc_dqn_fwd3_kernel(TcTrainParam
       tmem_st8(lane_base + kColAHi + 8 * cq, hi);
       tmem_st8(lane_base + kColALo + 8 * cq, lo);
       if (r < nrows) {   // the other two kernels read the gathered row instead of chasing the episode index again
-        float4* xo = reinterpret_cast<float4*>(p.xg + cur.dst * kMaxObsDim + 8 * cq);
+        float4* xo = reinterpret_cast<float4*>(p.xg + cur.dst * kTcObsDim + 8 * cq);
         xo[0] = make_float4(cur.x[0], cur.x[1], cur.x[2], cur.x[3]); xo[1] = make_float4(cur.x[4], cur.x[5], cur.x[6], cur.x[7]);
       }
     }
@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(kTrThreads, 1) tc_dqn_fwd3_kernel(TcTrainParam
 #pragma unroll
       for (int term = 0; term < 3; ++term)
 #pragma unroll
-        for (int ks = 0; ks < kMaxObsDim / 8; ++ks)
+        for (int ks = 0; ks < kTcObsDim / 8; ++ks)
           if (ks < k1steps) mma_tf32_ts(tmem + d_cur, tmem + (term == 0 ? kColALo : kColAHi) + ks * 8, (term == 1 ? dlo : dhi) + (uint32_t)((ks * 32) >> 4), idesc, (term | ks) ? 1u : 0u);
       mma_commit(bar);
       if (k > 0) {   // every thread is past the previous tile's TD head: publish its first row's outputs
@@ -541,7 +541,7 @@ __global__ void __launch_bounds__(kH3Threads, 1) tc_dh1w1_kernel(TcTrainParams p
         rc.g = __int_as_float(ga.x); rc.act = ga.y;
         rc.m1 = reinterpret_cast<const uint32_t*>(rp)[4 + cq];
         rc.m2 = reinterpret_cast<const uint32_t*>(rp)[8 + cq];
-        const float4* xp = reinterpret_cast<const float4*>(p.xg + rc.d * kMaxObsDim + 8 * cq);
+        const float4* xp = reinterpret_cast<const float4*>(p.xg + rc.d * kTcObsDim + 8 * cq);
         const float4 x0 = xp[0], x1 = xp[1];
         rc.x[0] = x0.x; rc.x[1] = x0.y; rc.x[2] = x0.z; rc.x[3] = x0.w; rc.x[4] = x1.x; rc.x[5] = x1.y; rc.x[6] = x1.z; rc.x[7] = x1.w;
 #pragma unroll
@@ -768,7 +768,7 @@ __global__ void __launch_bounds__(kH3Threads, 1) tc_dw2_kernel(TcTrainParams p) 
       if (cq < k1steps && vr0 + r < row_end) {
         int a, u, o;
         const size_t d = dst_of3(p.plan, p.src, net, vr0 + r, a, u, o);
-        const float4* xp = reinterpret_cast<const float4*>(p.xg + d * kMaxObsDim + 8 * cq);
+        const float4* xp = reinterpret_cast<const float4*>(p.xg + d * kTcObsDim + 8 * cq);
         const float4 x0 = xp[0], x1 = xp[1];
         x[0] = x0.x; x[1] = x0.y; x[2] = x0.z; x[3] = x0.w; x[4] = x1.x; x[5] = x1.y; x[6] = x1.z; x[7] = x1.w;
       }

@@ -20,6 +20,12 @@ from .. import _native as nat
 from ..lbf import TrajStore
 
 HIDDEN = 128
+MAX_IN_DIM = 128   # widest network input the learner kernels take (per-agent observation, or a centralised critic's joint observation)
+
+
+def check_in_dim(width, what):
+    if width > MAX_IN_DIM:
+        raise NotImplementedError(f"{what} is {width} wide; the learner kernels take at most {MAX_IN_DIM} input features")
 
 
 def _dim(space) -> int:
@@ -94,6 +100,7 @@ class QNetwork:
         if len(set(obs_dims)) != 1 or len(set(act_dims)) != 1:
             raise NotImplementedError("agents with different observation / action sizes are not implemented")
         self.in_dim, self.n_actions = obs_dims[0], act_dims[0]
+        check_in_dim(self.in_dim, "the observation")
         self.action_space = action_space
         self.agent_net = sharing_to_nets(parameter_sharing, self.n_agents)
         self.n_nets = max(self.agent_net) + 1
